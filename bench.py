@@ -26,6 +26,9 @@ than the 126 MB L2, so no flush is needed between timed iterations).
 
 `--impl reference` times the reference's CPU implementation of the path instead (the oracle port: the reference is Scala/JVM
 and cannot be built in this image), rank 0 only.
+
+`--dump-outputs DIR` writes, after the timed steps, the state table the last timed step left (rank 0's shard) as DIR/states.npy,
+so that two builds run with the same arguments (same seeded inputs) can be compared output for output.
 """
 from __future__ import annotations
 
@@ -51,11 +54,33 @@ ROUTED_EPA = 100
 ROUTED_SEED = 3
 NVLINK_PEAK_GBS = 770.0          # measured peer copy per direction per GPU on this pool (B200_PROFILING.md)
 M64 = (1 << 64) - 1
+DUMP_MAX_BYTES = 64_000_000      # --dump-outputs: all arrays together
 
 
 def algorithmic_bytes(n_agg: int, epa: int) -> int:
     """B_alg = stored event bytes + 8*(nAgg+1) CSR offsets + S*nAgg states written (SURVEY.md 8d)."""
     return n_agg * epa * 64 + 8 * (n_agg + 1) + STATE_BYTES * n_agg
+
+
+def state_columns(table):
+    """A Counter state table (u8 [n, 16], include/sgr.h) as float64 [n, 4]: count and version (the program's i32 words), then
+    the engine's u32 flags and err_idx. float64 holds every 32-bit value exactly."""
+    import numpy as np
+
+    table = np.ascontiguousarray(table)
+    cols = table.view(np.int32).astype(np.float64)
+    cols[:, 2:] = table.view(np.uint32)[:, 2:]
+    return cols
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes every array as out_dir/<name>.npy."""
+    import numpy as np
+
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_MAX_BYTES
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def measured_peak_gbs() -> tuple[float, str]:
@@ -187,9 +212,11 @@ def run_reference(args) -> None:
     t0 = time.perf_counter()
     nev = 0
     for _ in range(args.steps):
-        _, n, _ = O.fold_packed(O.MODEL_COUNTER, O.REC_FIXED64, placed, off, threads=cores, pinned=True)
+        states, n, _ = O.fold_packed(O.MODEL_COUNTER, O.REC_FIXED64, placed, off, threads=cores, pinned=True)
         nev += n
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"states": state_columns(states)})
     value = nev / dt
     sample = (f"{N_AGG} aggregates x {EVENTS_PER_AGG} events per step (the full configs[1] log, host memory first-touched by the "
               f"pinned worker that folds it), {args.steps} steps")
@@ -568,7 +595,11 @@ def main() -> None:
     ap.add_argument("--no-configs", action="store_true", help="skip configs[0], [3], [4] (N = 1)")
     ap.add_argument("--scale", type=float, default=1.0, help="shrink configs[2] and configs[3] (debugging on a busy box); 1.0 = the BASELINE sizes")
     ap.add_argument("--routed-iters", type=int, default=3)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the state table of the last one as "
+                    "DIR/states.npy: float64 [aggregates, 4] = count, version, flags, err_idx (rank 0's shard)")
     args = ap.parse_args()
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)   # an unusable DIR fails here, not after the run
     if args.impl == "reference":
         run_reference(args)
         return
@@ -786,6 +817,9 @@ def main() -> None:
     wire.clear()
     pinned = None
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        # timed region 1's table: nothing has folded on `eng` since its last step
+        dump_outputs(args.dump_outputs, {"states": state_columns(eng.states_tensor().cpu().numpy())})
     e2.close(); eng.close()
     cpu_rec = np.array(host_log_np, copy=True) if (world == 1 and not args.no_cpu_baseline) else None
     del rec, host_log, host_log_np

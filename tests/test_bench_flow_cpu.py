@@ -87,3 +87,20 @@ def test_wire_section_leaves_a_result_on_every_path():
             sys.modules["surge_b200.dingest"] = saved
         else:
             sys.modules.pop("surge_b200.dingest", None)
+
+
+def test_dumped_state_columns_keep_every_32_bit_word(tmp_path):
+    """--dump-outputs: count and version are signed, flags and err_idx unsigned, all exact in float64, and the file reads back."""
+    import pytest
+    import bench
+
+    tab = np.zeros((3, 16), dtype=np.uint8)
+    tab.view(np.int32)[0] = [-(1 << 31), 7, 3, 0]
+    tab.view(np.uint32)[1] = [0xFFFFFFFF, 1 << 31, 0xFFFFFFFF, 5]
+    cols = bench.state_columns(tab)
+    assert cols.dtype == np.float64
+    assert cols.tolist() == [[-(1 << 31), 7, 3, 0], [-1, -(1 << 31), 0xFFFFFFFF, 5], [0, 0, 0, 0]]
+    bench.dump_outputs(str(tmp_path), {"states": cols})
+    assert np.array_equal(np.load(tmp_path / "states.npy"), cols)
+    with pytest.raises(AssertionError):
+        bench.dump_outputs(str(tmp_path), {"states": np.zeros(bench.DUMP_MAX_BYTES // 8 + 1)})
