@@ -208,7 +208,11 @@ int32_t sgr_load_events_indexed_device(sgr_engine* e, const void* d_events, uint
 
 /* Load records in ARRIVAL order (a Kafka partition log interleaves aggregates) and group
  * them, stably, by aggregate index into CSR form on the device. n_agg is the number of
- * dense aggregate indices (records carry agg < n_agg). Fixed 64-byte records only. */
+ * dense aggregate indices (records carry agg < n_agg). Fixed 64-byte records only.
+ * Holes: a record with agg == UINT64_MAX is a hole (what the device ingest leaves in place of a dropped record) and is
+ * skipped by every arrival-order entry point (sgr_load_unsorted*, sgr_fold_unsorted*, sgr_fold_incremental*): the outcome,
+ * statistics included, is that of the same records without the holes. Any other agg >= n_agg fails the call with
+ * SGR_ERR_INVALID and nothing is applied. */
 int32_t sgr_load_unsorted(sgr_engine* e, const void* records, uint64_t n_records, uint64_t n_agg);
 int32_t sgr_load_unsorted_device(sgr_engine* e, const void* d_records, uint64_t n_records, uint64_t n_agg);
 
@@ -233,9 +237,12 @@ int32_t sgr_fold(sgr_engine* e);
 int32_t sgr_fold_async(sgr_engine* e);
 int32_t sgr_wait(sgr_engine* e);
 
-/* Append one micro-batch (arrival order, fixed records) to the live state table: group by
+/* Append one micro-batch (arrival order, fixed records, holes skipped) to the live state table: group by
  * aggregate, fold onto the current states, write back (PersistentActor.doApplyEvent on a
- * live actor, PersistentActor.scala:245-264). Requires a prior fold or set_initial_states. */
+ * live actor, PersistentActor.scala:245-264). Requires a prior fold or set_initial_states.
+ * A fold that fails half-applied (more throwing aggregates than the replay list holds on an in-place fold) invalidates the
+ * table: reads, sgr_grow_states, sgr_fold_ingested and sgr_dingest_fold fail with SGR_ERR_STATE until sgr_set_initial_states
+ * (NULL included), a full fold or sgr_fold_unsorted replaces it. */
 int32_t sgr_fold_incremental(sgr_engine* e, const void* records, uint64_t n_records);
 int32_t sgr_fold_incremental_device(sgr_engine* e, const void* d_records, uint64_t n_records);
 
@@ -251,6 +258,9 @@ int32_t sgr_get(sgr_engine* e, const uint8_t* key, uint32_t klen,
                 void* out, uint32_t cap, uint32_t* outlen, int32_t* exists);
 int32_t sgr_get_index(sgr_engine* e, uint64_t agg, void* out, uint32_t cap,
                       uint32_t* outlen, int32_t* exists, uint32_t* flags, uint32_t* err_idx);
+/* The dense aggregate index sgr_get resolves an id to (*agg = UINT64_MAX for an unknown id). The device ingest hands out
+ * indices from an atomic counter, so this is how a caller reaches an id's flags and err_idx through sgr_get_index. */
+int32_t sgr_key_index(sgr_engine* e, const uint8_t* key, uint32_t klen, uint64_t* agg);
 
 /* Export the whole state table (n_agg * state_bytes) and, optionally, bitmaps
  * (bit i of byte i/8, LSB first). Any out pointer may be NULL. */
@@ -458,7 +468,7 @@ int32_t sgr_append_keys(sgr_engine* e, const void* owner, const uint8_t* keys, c
  * read_committed bookkeeping (control batches, aborted transactions, partition positions). csrc/ingest.cpp is its checker
  * (tests/test_gpu_dingest.py: identical states, ids, offsets and statistics on the same bytes).
  *   - value framing: SGR_VALUE_PACKED only (protobuf / JSON values: use the host ingest);
- *   - programs in the sort-free class (16-byte state, class 0): dropped records stay in place as holes the fold skips;
+ *   - dropped records (markers, duplicates, null values) stay in place as holes (aggregate index UINT64_MAX) the fold skips;
  *   - dense indices are stable per id but follow no arrival-order promise (they come from an atomic counter);
  *   - polls are processed in groups of SGR_DINGEST_GROUP (default 8192) batches, each group one chain of launches on one of eight
  *     streams; batches decompress into an arena of 3x the wire bytes (a poll that compresses better is decoded a second time from

@@ -117,7 +117,7 @@ __device__ __forceinline__ void apply_rec(const RecView& r, uint32_t idx1, uint3
   if (COMPACT) { slot = r.q0.x; type = r.q0.y >> 27; idx1 = ib + (r.q0.y & 0x07ffffffu); }
   else if (a.src.carried) { slot = r.q0.z; type = r.q0.x; idx1 = ib + r.q0.w; }
   else { slot = ((unsigned long long)r.q0.w << 32) | r.q0.z; type = r.q0.x; }
-  if (slot == ~0ull) return;   // a hole: a record the device decode dropped in place (flush marker, duplicate, null value)
+  if (slot == ~0ull) { atomicAdd(a.counters + 0, 1ull); return; }   // a hole: a record the device decode dropped in place (flush marker, duplicate, null value)
   if (slot >= a.n_slots) { atomicAdd(a.counters + 4, 1ull); return; }
   uint8_t* entry = a.scr + (slot << a.lay.entry_shift);
   const uint32_t fl = type < 16u ? tab[type * kTabStride] : 0u;

@@ -50,7 +50,7 @@ struct BulkSrc {
   uint32_t rec_bytes;             // record stride
 };
 
-// counters (u64): [0] records seen [1] throwing slots (after finish) [3] error list length [4] records with slot >= n_slots
+// counters (u64): [0] holes (agg == UINT64_MAX, skipped) [1] throwing slots (after finish) [3] error list length [4] records with slot >= n_slots
 cudaError_t launch_bulk_accumulate(const BulkSrc& src, uint64_t n_slots, void* d_scratch, const RowProgram& prog, const BulkLayout& lay,
                                    unsigned long long* d_counters, int num_sms, cudaStream_t st);
 // by slot: applies (last, accumulators) to the prior state, sets EXISTS/CHANGED, zeroes the slot's scratch; slots that saw a

@@ -134,6 +134,7 @@ struct sgr_dingest {
   uint64_t slots = 0, max_keys = 0, arena_cap = 0;
   uint64_t keys_on_host = 0;                // ids already appended to the engine's key table
   uint64_t id_bytes_on_host = 0;            // ... and the id-arena bytes they occupy
+  uint64_t keys_reported = 0;               // ids counted in the n_new_keys of a successful poll
   cudaEvent_t keys_landed = nullptr;
   uint64_t generation = 0;                  // bumped by sgr_dingest_reset: a new dictionary is a new owner of the engine's key table
   void* h_ctl = nullptr;                    // page-locked landing area
@@ -574,7 +575,7 @@ int32_t sgr_dingest_fold(sgr_dingest* g, sgr_ingest_stats* stats) {
       const int32_t rc = dfail(g, SGR_ERR_CAPACITY, "device id dictionary full (%llu ids / %llu id bytes allowed): create the device ingest with larger bounds", (unsigned long long)g->max_keys, (unsigned long long)g->arena_cap);
       discard_poll(g); return rc;
     }
-    st.n_markers = h[2]; st.n_null_values = h[3]; st.n_duplicates += h[4]; st.n_records = h[6]; st.n_new_keys = h[0] - g->keys_on_host;   // (ids a failed poll interned become visible with the next good one)
+    st.n_markers = h[2]; st.n_null_values = h[3]; st.n_duplicates += h[4]; st.n_records = h[6]; st.n_new_keys = h[0] - g->keys_reported;   // (ids a failed poll interned are counted by the next good one)
     // ---- grow the table for the new ids, hand their names to the engine's key table, fold
     const uint64_t n_keys = h[0];
     void* d_states = nullptr; uint64_t n_agg = 0; uint32_t sb = 0;
@@ -626,9 +627,11 @@ int32_t sgr_dingest_fold(sgr_dingest* g, sgr_ingest_stats* stats) {
     int32_t rc_fold = SGR_OK;
     if (nrec) rc_fold = sgr_fold_incremental_device(g->eng, g->out.b.p, nrec);
     if (appender.joinable()) appender.join();
+    // the engine's key table holds these ids now, whatever the fold returned: the next poll appends only what follows them
+    if (rc_append == SGR_OK) { g->keys_on_host = n_keys; g->id_bytes_on_host = h[1]; }
     if (rc_fold) { dfail(g, rc_fold, "engine: %s", sgr_last_error(g->eng)); discard_poll(g); return rc_fold; }
     if (rc_append) { dfail(g, rc_append, "engine: %s", sgr_last_error(g->eng)); discard_poll(g); return rc_append; }
-    g->keys_on_host = n_keys; g->id_bytes_on_host = h[1];
+    g->keys_reported = n_keys;
   }
   lap(4);
   g->ms[5] = std::chrono::duration<float, std::milli>(Clk::now() - t_begin).count();
@@ -648,7 +651,7 @@ int32_t sgr_dingest_fold(sgr_dingest* g, sgr_ingest_stats* stats) {
 int32_t sgr_dingest_reset(sgr_dingest* g) {
   if (!g) return SGR_ERR_INVALID;
   discard_poll(g);
-  g->parts.clear(); g->staged.clear(); g->total = sgr_ingest_stats{}; g->keys_on_host = 0; g->id_bytes_on_host = 0; ++g->generation;
+  g->parts.clear(); g->staged.clear(); g->total = sgr_ingest_stats{}; g->keys_on_host = 0; g->id_bytes_on_host = 0; g->keys_reported = 0; ++g->generation;
   DG_TRY(g, cudaMemsetAsync(g->tags.p, 0, g->slots * 8, g->stream));
   DG_TRY(g, cudaMemsetAsync(g->slot_idx.p, 0, g->slots * 4, g->stream));
   DG_TRY(g, cudaMemsetAsync(g->ctl.p, 0, 9 * 8, g->stream));                                  // ([9], the arena's capacity, stays)

@@ -62,6 +62,8 @@ struct sgr_engine {
 
   DevBuf states;        // n_agg * state_bytes, live table
   bool states_valid = false;  // holds prior states (set_initial_states or a previous fold)
+  bool states_invalidated = false;  // a failed in-place fold left the table half-applied: nothing may fold onto it (or grow it)
+                                    // until set_initial_states, a full fold or fold_unsorted replaces it
   uint64_t states_n = 0;
   DevBuf counters;      // 8 x u64
   GroupScratch group;   // K5 scratch
@@ -415,7 +417,7 @@ int32_t finish_fold(sgr_engine* e) {
     if (e->pending_prior) {
       // the kernel has already overwritten the non-throwing aggregates in place: the table is half-applied. It must not be
       // served, and a retry must not double-apply — invalidate it (reads fail with SGR_ERR_STATE until the next full fold)
-      e->states_valid = false; mark_dirty(e);
+      e->states_valid = false; e->states_invalidated = true; mark_dirty(e);
       return fail(e, SGR_ERR_UNSUPPORTED, "replay list overflow on an in-place incremental fold: state table invalidated, rebuild it");
     }
     CUDA_TRY(e, cudaMemsetAsync(e->counters.p, 0, 64, e->stream));
@@ -428,6 +430,7 @@ int32_t finish_fold(sgr_engine* e) {
     CUDA_TRY(e, cudaStreamSynchronize(e->stream));
     float ms2 = 0; CUDA_TRY(e, cudaEventElapsedTime(&ms2, e->ev2, e->ev3));
     e->stats.ms_fold += ms2; e->stats.fold_launches += 1;
+    e->pending_used_rows = false;   // h now holds the sequential kernel's counts
   }
   const uint64_t n_seg = e->pending_n_seg;
   e->stats.n_aggregates = n_seg;
@@ -600,15 +603,16 @@ static int32_t load_unsorted_impl(sgr_engine* e, const void* d_records, uint64_t
   CUDA_TRY(e, e->own_events.reserve(n_records * 64));
   CUDA_TRY(e, e->own_offsets.reserve((n_agg + 1) * 8));
   CUDA_TRY(e, cudaEventRecord(e->ev0, e->stream));
-  unsigned long long bad = 0;
+  unsigned long long bad = 0, holes = 0;
   cudaError_t ce = group_by_agg_stable(e->group, (const uint8_t*)d_records, n_records, n_agg, (uint8_t*)e->own_events.p,
-                                       (uint64_t*)e->own_offsets.p, nullptr, nullptr, (unsigned long long*)e->counters.p, e->stream, &bad);
+                                       (uint64_t*)e->own_offsets.p, nullptr, nullptr, (unsigned long long*)e->counters.p, e->stream, &bad, &holes);
   if (ce != cudaSuccess) return fail(e, SGR_ERR_CUDA, "group-by: %s", cudaGetErrorString(ce));
   CUDA_TRY(e, cudaEventRecord(e->ev1, e->stream));
   CUDA_TRY(e, cudaStreamSynchronize(e->stream));
   CUDA_TRY(e, cudaEventElapsedTime(&e->stats.ms_group, e->ev0, e->ev1));
   if (bad) return fail(e, SGR_ERR_INVALID, "%llu records carry an aggregate index >= n_agg", bad);
-  return after_load(e, (const uint8_t*)e->own_events.p, (const uint64_t*)e->own_offsets.p, n_records * 64, n_agg);
+  // the holes were sorted behind the last segment: the log ends before them
+  return after_load(e, (const uint8_t*)e->own_events.p, (const uint64_t*)e->own_offsets.p, (n_records - holes) * 64, n_agg);
 }
 
 int32_t sgr_load_unsorted_device(sgr_engine* e, const void* d_records, uint64_t n_records, uint64_t n_agg) {
@@ -639,12 +643,12 @@ int32_t sgr_set_initial_states(sgr_engine* e, const void* states, uint64_t n_agg
   if (!e) return SGR_ERR_INVALID;
   if (!e->has_program) return fail(e, SGR_ERR_NO_PROGRAM, "register a fold program first");
   // NULL only says "the next fold starts from None everywhere": no device work, no wait
-  if (!states) { e->states_valid = false; mark_dirty(e); return SGR_OK; }
+  if (!states) { e->states_valid = false; e->states_invalidated = false; mark_dirty(e); return SGR_OK; }
   int32_t rc = before_load(e); if (rc) return rc;
   rc = ensure_states(e, n_agg); if (rc) return rc;
   CUDA_TRY(e, cudaMemcpyAsync(e->states.p, states, (size_t)n_agg * e->program.state_bytes, cudaMemcpyHostToDevice, e->stream));
   CUDA_TRY(e, cudaStreamSynchronize(e->stream));
-  e->states_valid = true;
+  e->states_valid = true; e->states_invalidated = false;
   e->inc_atomic_prev_valid = false; e->inc_prev_n = 0;
   mark_dirty(e);
   return SGR_OK;
@@ -660,6 +664,7 @@ static int32_t fold_begin(sgr_engine* e, bool pipelined) {
   if (!pipelined) { rc = finish_fold(e); if (rc) return rc; }
   const bool prior = e->states_valid && e->states_n == e->n_agg;
   rc = ensure_states(e, e->n_agg); if (rc) return rc;
+  e->states_invalidated = false;   // a full fold replaces the table (a failed in-place fold left prior states invalid)
   rc = enqueue_fold(e, e->d_events, e->d_offsets, nullptr, e->n_agg, prior, e->event_bytes, e->offsets_aligned64, e->log_begin, e->log_end);
   if (rc) return rc;
   e->states_valid = true;
@@ -734,7 +739,7 @@ static int32_t fold_incremental_atomic(sgr_engine* e, const void* d_records, uin
   e->inc_flip ^= 1;
   e->inc_prev_n = 0;
   e->stats.ms_group = 0;
-  e->stats.n_aggregates = h[5]; e->stats.n_errors = h[1]; e->stats.n_events = n_records - h[6];
+  e->stats.n_aggregates = h[5]; e->stats.n_errors = h[1]; e->stats.n_events = n_records - h[0] - h[6];   // [0] holes
   e->stats.event_bytes = n_records * 64; e->stats.n_long_segments = 0;
   e->stats.algorithmic_bytes = n_records * 64 + 2 * (uint64_t)e->program.state_bytes * h[5];
   e->stats.fold_launches = 1;
@@ -759,16 +764,17 @@ static int32_t fold_incremental_impl(sgr_engine* e, const void* d_records, uint6
   // per-batch flags (CHANGED/ERROR) of the aggregates touched by the previous batch are cleared
   if (e->inc_prev_n) clear_batch_flags((uint8_t*)e->states.p, e->program.state_bytes, (const uint32_t*)e->inc_prev_ids.p, e->inc_prev_n, e->stream);
   else clear_batch_flags((uint8_t*)e->states.p, e->program.state_bytes, nullptr, n_agg, e->stream);
-  unsigned long long bad = 0;
+  unsigned long long bad = 0, holes = 0;
   uint64_t n_touched = 0;
   cudaError_t ce = group_by_agg_stable(e->group, (const uint8_t*)d_records, n_records, n_agg, (uint8_t*)grouped.p,
                                        (uint64_t*)e->inc_offsets.p, (uint32_t*)e->inc_ids.p, &n_touched,
-                                       (unsigned long long*)e->counters.p, e->stream, &bad);
+                                       (unsigned long long*)e->counters.p, e->stream, &bad, &holes);
   if (ce != cudaSuccess) return fail(e, SGR_ERR_CUDA, "group-by: %s", cudaGetErrorString(ce));
   CUDA_TRY(e, cudaEventRecord(e->ev3, e->stream));
   if (bad) return fail(e, SGR_ERR_INVALID, "%llu records carry an aggregate index >= n_agg", bad);
+  const uint64_t real_bytes = (n_records - holes) * 64;   // the holes were sorted behind the last segment
   int32_t rc = enqueue_fold(e, (const uint8_t*)grouped.p, (const uint64_t*)e->inc_offsets.p, (const uint32_t*)e->inc_ids.p, n_touched, true,
-                            n_records * 64, true, 0, n_records * 64);
+                            real_bytes, true, 0, real_bytes);
   if (rc) return rc;
   rc = finish_fold(e); if (rc) return rc;
   CUDA_TRY(e, cudaEventElapsedTime(&e->stats.ms_group, e->ev2, e->ev3));
@@ -816,6 +822,7 @@ int32_t sgr_grow_states(sgr_engine* e, uint64_t n_agg) {
   if (!e->has_program) return fail(e, SGR_ERR_NO_PROGRAM, "register a fold program first");
   int32_t rc = use_device(e); if (rc) return rc;
   rc = before_load(e); if (rc) return rc;
+  if (e->states_invalidated) return fail(e, SGR_ERR_STATE, "state table invalidated by a failed fold: reset it (set_initial_states) or rebuild it");
   if (e->states_valid && n_agg <= e->states_n) return SGR_OK;
   const size_t sb = e->program.state_bytes;
   if (!e->states_valid && e->states.p && e->states.cap >= (size_t)n_agg * sb) {
@@ -880,6 +887,7 @@ int32_t sgr_fold_ingested(sgr_engine* e, sgr_ingest* g) {
   OpLock op_lock(e);
   if (!e || !g) return fail(e, SGR_ERR_INVALID, "null argument");
   { int32_t rc0 = use_device(e); if (rc0) return rc0; }
+  if (e->states_invalidated) return fail(e, SGR_ERR_STATE, "state table invalidated by a failed fold: reset it (set_initial_states) or rebuild it");
   // from now on the ingest decodes straight into page-locked memory (what is pending right now is moved once)
   if (sgr_ingest_set_allocator(g, pinned_alloc, pinned_free)) return fail(e, SGR_ERR_OOM, "ingest: %s", sgr_ingest_last_error(g));
   const void* recs = nullptr; uint64_t n_records = 0;
@@ -922,8 +930,8 @@ int32_t sgr_get_index(sgr_engine* e, uint64_t agg, void* out, uint32_t cap, uint
   return SGR_OK;
 }
 
-int32_t sgr_get(sgr_engine* e, const uint8_t* key, uint32_t klen, void* out, uint32_t cap, uint32_t* outlen, int32_t* exists) {
-  if (!e || (!key && klen)) return fail(e, SGR_ERR_INVALID, "null argument");
+// dense index of an aggregate id in the key table (rebuilt first if ids were appended since), or -1
+static int32_t find_key(sgr_engine* e, const uint8_t* key, uint32_t klen, int64_t* idx) {
   if (e->keys_stale.load(std::memory_order_acquire)) {
     std::lock_guard<std::mutex> lk(e->keys_mu);
     if (e->keys_stale.load(std::memory_order_relaxed)) {
@@ -935,7 +943,22 @@ int32_t sgr_get(sgr_engine* e, const uint8_t* key, uint32_t klen, void* out, uin
     }
   }
   std::shared_ptr<const KeyTable> kt = std::atomic_load(&e->keys);
-  int64_t idx = kt ? kt->find(key, klen) : -1;
+  *idx = kt ? kt->find(key, klen) : -1;
+  return SGR_OK;
+}
+
+int32_t sgr_key_index(sgr_engine* e, const uint8_t* key, uint32_t klen, uint64_t* agg) {
+  if (!e || (!key && klen) || !agg) return fail(e, SGR_ERR_INVALID, "null argument");
+  int64_t idx = -1;
+  int32_t rc = find_key(e, key, klen, &idx); if (rc) return rc;
+  *agg = idx < 0 ? UINT64_MAX : (uint64_t)idx;
+  return SGR_OK;
+}
+
+int32_t sgr_get(sgr_engine* e, const uint8_t* key, uint32_t klen, void* out, uint32_t cap, uint32_t* outlen, int32_t* exists) {
+  if (!e || (!key && klen)) return fail(e, SGR_ERR_INVALID, "null argument");
+  int64_t idx = -1;
+  { int32_t rc = find_key(e, key, klen, &idx); if (rc) return rc; }
   if (idx < 0) {  // unknown aggregate id: Option.empty, like a KTable miss
     if (exists) *exists = 0;
     if (outlen) *outlen = 0;
@@ -1016,7 +1039,7 @@ static int32_t replay_throwing_slots(sgr_engine* e, const void* d_records, uint6
   CUDA_TRY(e, e->inc_offsets.reserve((n_agg + 2) * 8));
   unsigned long long bad = 0;
   cudaError_t ce = group_by_agg_stable(e->group, (const uint8_t*)d_records, n_records, n_agg, (uint8_t*)grouped.p, (uint64_t*)e->inc_offsets.p,
-                                       nullptr, nullptr, (unsigned long long*)e->counters.p, e->stream, &bad);
+                                       nullptr, nullptr, (unsigned long long*)e->counters.p, e->stream, &bad, nullptr);
   if (ce != cudaSuccess) return fail(e, SGR_ERR_CUDA, "group-by (replay): %s", cudaGetErrorString(ce));
   CUDA_TRY(e, cudaMemsetAsync(e->counters.p, 0, 64, e->stream));
   FoldArgs a{};
@@ -1065,7 +1088,7 @@ static int32_t fold_bulk(sgr_engine* e, const uint8_t* d_records, uint64_t n_rec
   unsigned long long throwing = 0, dropped = 0;
   if (h[3]) { rc = replay_throwing_slots(e, d_records, n_records, n_agg, (const uint32_t*)e->bulk_err_ids.p, h[3], &throwing, &dropped); if (rc) return rc; }
   e->stats.ms_group = 0;
-  e->stats.n_aggregates = n_agg; e->stats.n_errors = throwing; e->stats.n_events = n_records - dropped;
+  e->stats.n_aggregates = n_agg; e->stats.n_errors = throwing; e->stats.n_events = n_records - h[0] - dropped;   // [0] holes
   e->stats.event_bytes = n_records * 64; e->stats.n_long_segments = 0;
   e->stats.algorithmic_bytes = n_records * 64 + (uint64_t)(16 + 2 * e->program.state_bytes) * n_agg;
   e->stats.fold_launches = 2;
@@ -1083,7 +1106,7 @@ static int32_t fold_arrival_order(sgr_engine* e, const uint8_t* d_records, uint6
   if (sort_free) {
     rc = ensure_states(e, n_agg); if (rc) return rc;
     CUDA_TRY(e, cudaMemsetAsync(e->states.p, 0, (size_t)n_agg * e->program.state_bytes, e->stream));
-    e->states_valid = true;
+    e->states_valid = true; e->states_invalidated = false;
     e->loaded = false;
     if (e->bulk_ok && e->opt_bulk && n_records < (1ull << 30)) {
       e->inc_atomic_prev_valid = false; e->inc_prev_n = 0;   // the next micro-batch clears every slot's per-batch flags
@@ -1196,7 +1219,7 @@ int32_t sgr_dist_route_and_fold(sgr_engine* e, const void* d_records, uint64_t n
     rc = ensure_states(e, n_local); if (rc) return rc;
     rc = ensure_bulk_buffers(e, n_local); if (rc) return rc;
     CUDA_TRY(e, cudaMemsetAsync(e->states.p, 0, (size_t)n_local * e->program.state_bytes, e->stream));
-    e->states_valid = true; e->loaded = false; e->inc_atomic_prev_valid = false; e->inc_prev_n = 0;
+    e->states_valid = true; e->states_invalidated = false; e->loaded = false; e->inc_atomic_prev_valid = false; e->inc_prev_n = 0;
     PushFoldArgs pf{};
     pf.prog = &e->row_prog; pf.lay = &e->bulk_lay; pf.scratch = e->bulk_scratch.p; pf.states = (uint8_t*)e->states.p;
     pf.err_ids = (uint32_t*)e->bulk_err_ids.p; pf.counters = (unsigned long long*)e->bulk_counters.p; pf.n_slots = n_local;

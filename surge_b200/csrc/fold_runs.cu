@@ -59,7 +59,12 @@ template <int W, int CLS = 1>
 __device__ __forceinline__ Xf<W> compose(const Xf<W>& a, const Xf<W>& b) {
   // class 1: b.ex == 0 means b holds only IF_EXISTS events (or nothing); they apply iff the state exists after a — a
   // tombstoned prefix absorbs them. (In class 0, b.ex == 0 only for the identity, where the plain rule gives a too.)
-  if (CLS == 1 && b.ex == 0u && a.ex == EX_NONE) return a;
+  // A throwing event sets no exists-op either: its error bit must survive, or the segment is never replayed.
+  if (CLS == 1 && b.ex == 0u && a.ex == EX_NONE) {
+    Xf<W> r = a;
+    r.m |= b.m & M_ERR;
+    return r;
+  }
   Xf<W> r;
   r.m = a.m | b.m;
   r.ex = b.ex ? b.ex : a.ex;

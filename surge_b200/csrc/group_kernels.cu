@@ -25,11 +25,14 @@ constexpr int kPerWarp = kTile / kWarps;  // 512 keys per warp
 constexpr int kRounds = kPerWarp / 32;    // 16
 
 // ---------------------------------------------------------------- keys
+// A hole (agg == UINT64_MAX: a record the device decode dropped in place) gets the sentinel key n_agg, which sorts after every
+// real key; any other agg >= n_agg is counted as bad.
 __global__ void extract_keys_kernel(const uint8_t* __restrict__ rec, uint32_t n, uint64_t n_agg,
-                                    uint32_t* __restrict__ keys, unsigned long long* __restrict__ bad) {
+                                    uint32_t* __restrict__ keys, unsigned long long* __restrict__ bad, unsigned long long* __restrict__ holes) {
   const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const unsigned long long agg = *reinterpret_cast<const unsigned long long*>(rec + (size_t)i * 64 + 8);
+  if (agg == ~0ull) { atomicAdd(holes, 1ull); keys[i] = (uint32_t)n_agg; return; }
   if (agg >= n_agg) atomicAdd(bad, 1ull);
   keys[i] = (uint32_t)agg;
 }
@@ -192,7 +195,7 @@ __global__ void __launch_bounds__(kThreads) radix_scatter_kernel(const uint32_t*
 }
 
 // ---------------------------------------------------------------- CSR offsets from sorted keys
-// full mode: offsets[a] = 64 * lower_bound(sorted, a) for a in [0, n_agg]
+// full mode: offsets[a] = 64 * lower_bound(sorted, a) for a in [0, n_agg] (the holes' sentinel run starts at offsets[n_agg])
 __global__ void offsets_full_kernel(const uint32_t* __restrict__ sorted, uint32_t n, uint64_t n_agg, uint64_t* __restrict__ offsets) {
   const uint64_t a = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (a > n_agg) return;
@@ -204,7 +207,7 @@ __global__ void offsets_full_kernel(const uint32_t* __restrict__ sorted, uint32_
   offsets[a] = (uint64_t)lo * 64;
 }
 
-// compact mode: heads[j] = 1 where a new aggregate starts in the sorted order
+// compact mode: heads[j] = 1 where a new aggregate (or the holes' sentinel run, which comes last) starts in the sorted order
 __global__ void heads_kernel(const uint32_t* __restrict__ sorted, uint32_t n, uint32_t* __restrict__ heads) {
   const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= n) return;
@@ -212,9 +215,14 @@ __global__ void heads_kernel(const uint32_t* __restrict__ sorted, uint32_t n, ui
 }
 __global__ void compact_kernel(const uint32_t* __restrict__ sorted, uint32_t n, const uint32_t* __restrict__ heads,
                                const uint32_t* __restrict__ pos, uint32_t* __restrict__ ids, uint64_t* __restrict__ offsets,
-                               unsigned long long* __restrict__ n_touched) {
+                               uint32_t hole_key, unsigned long long* __restrict__ n_touched) {
   const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= n) return;
+  if (sorted[j] == hole_key) {
+    // the holes' run ends the real records: no touched id of its own
+    if (heads[j]) { offsets[pos[j]] = (uint64_t)j * 64; *n_touched = pos[j]; }
+    return;
+  }
   if (heads[j]) { ids[pos[j]] = sorted[j]; offsets[pos[j]] = (uint64_t)j * 64; }
   if (j == n - 1) {
     const uint32_t t = pos[j] + heads[j];
@@ -259,10 +267,11 @@ void clear_batch_flags(uint8_t* d_states, uint32_t state_bytes, const uint32_t* 
 cudaError_t group_by_agg_stable(GroupScratch& sc, const uint8_t* d_records, uint64_t n64, uint64_t n_agg,
                                 uint8_t* d_out_records, uint64_t* d_out_offsets, uint32_t* d_touched_ids,
                                 uint64_t* n_touched, unsigned long long* d_counters, cudaStream_t st,
-                                unsigned long long* bad_out) {
+                                unsigned long long* bad_out, unsigned long long* holes_out) {
   const uint32_t n = (uint32_t)n64;
   cudaError_t e;
   *bad_out = 0;
+  if (holes_out) *holes_out = 0;
   if (n_touched) *n_touched = 0;
   if (n == 0) {
     // empty batch: every aggregate has an empty segment
@@ -282,10 +291,11 @@ cudaError_t group_by_agg_stable(GroupScratch& sc, const uint8_t* d_records, uint
   uint32_t* tmp = (uint32_t*)sc.scan_tmp.p;
 
   if ((e = cudaMemsetAsync(d_counters, 0, 64, st)) != cudaSuccess) return e;
-  extract_keys_kernel<<<cdiv(n, 256), 256, 0, st>>>(d_records, n, n_agg, ka, d_counters + 4);
+  extract_keys_kernel<<<cdiv(n, 256), 256, 0, st>>>(d_records, n, n_agg, ka, d_counters + 4, d_counters + 6);
 
+  // keys 0..n_agg (n_agg: the holes' sentinel) must all be told apart, or a hole lands in slot n_agg-1's bucket
   int bits = 1;
-  while (bits < 32 && (1ull << bits) < n_agg) ++bits;
+  while (bits < 32 && (1ull << bits) <= n_agg) ++bits;
   for (int shift = 0; shift < bits; shift += 8) {
     radix_hist_kernel<<<nblocks, kThreads, 0, st>>>(ka, n, shift, hist, nblocks);
     if ((e = exclusive_scan_u32(hist, hist, 256 * nblocks, tmp, st)) != cudaSuccess) return e;
@@ -304,14 +314,15 @@ cudaError_t group_by_agg_stable(GroupScratch& sc, const uint8_t* d_records, uint
     uint32_t* pos = heads + n;
     heads_kernel<<<cdiv(n, 256), 256, 0, st>>>(ka, n, heads);
     if ((e = exclusive_scan_u32(heads, pos, n, tmp, st)) != cudaSuccess) return e;
-    compact_kernel<<<cdiv(n, 256), 256, 0, st>>>(ka, n, heads, pos, d_touched_ids, d_out_offsets, d_counters + 5);
+    compact_kernel<<<cdiv(n, 256), 256, 0, st>>>(ka, n, heads, pos, d_touched_ids, d_out_offsets, (uint32_t)n_agg, d_counters + 5);
   }
   gather_records_kernel<<<cdiv((uint64_t)n * 4, 256), 256, 0, st>>>(d_records, ia, n, d_out_records);
   if ((e = cudaGetLastError()) != cudaSuccess) return e;
-  unsigned long long h[2];
-  if ((e = cudaMemcpyAsync(h, d_counters + 4, 16, cudaMemcpyDeviceToHost, st)) != cudaSuccess) return e;
+  unsigned long long h[3];
+  if ((e = cudaMemcpyAsync(h, d_counters + 4, 24, cudaMemcpyDeviceToHost, st)) != cudaSuccess) return e;
   if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return e;
   *bad_out = h[0];
+  if (holes_out) *holes_out = h[2];
   if (n_touched) *n_touched = h[1];
   return cudaSuccess;
 }

@@ -76,7 +76,7 @@ struct IncArgs {
   Scratch* scr; uint8_t* states;
   uint32_t* touched_ids; uint32_t* err_ids;
   const uint32_t* prev_ids; const unsigned long long* prev_n;   // previous batch's touched list (prev_n may be null)
-  unsigned long long* counters;  // [1] throwing slots [3] error list [4] bad records [5] touched [6] dropped events [7] barrier
+  unsigned long long* counters;  // [0] holes [1] throwing slots [3] error list [4] bad records [5] touched [6] dropped events [7] barrier
   uint32_t fast2;                    // every state word is add-only or set-only across the program: phases A and B fuse
   uint32_t set_only_mask;            // bit w: word w is only ever SET (otherwise, in fast2 mode, only ever ADDed)
   unsigned long long replay_budget;  // phase D runs only if n_err * n <= budget (it re-scans the batch per throwing slot); beyond
@@ -108,7 +108,7 @@ __global__ void __launch_bounds__(256) inc_fused_kernel(const __grid_constant__ 
     for (uint64_t i = tid; i < a.n; i += nthreads) {
       const uint8_t* r = a.rec + i * 64;
       const unsigned long long slot = *reinterpret_cast<const unsigned long long*>(r + 8);
-      if (slot == ~0ull) continue;   // hole left by the device decode
+      if (slot == ~0ull) { atomicAdd(a.counters + 0, 1ull); continue; }   // hole left by the device decode
       if (slot >= a.n_slots) { atomicAdd(a.counters + 4, 1ull); continue; }
       uint32_t* sw = reinterpret_cast<uint32_t*>(a.scr + slot);
       unsigned long long* s64 = reinterpret_cast<unsigned long long*>(sw + 2);
@@ -161,7 +161,7 @@ __global__ void __launch_bounds__(256) inc_fused_kernel(const __grid_constant__ 
   for (uint64_t i = tid; i < a.n; i += nthreads) {
     const uint8_t* r = a.rec + i * 64;
     const unsigned long long slot = *reinterpret_cast<const unsigned long long*>(r + 8);
-    if (slot == ~0ull) continue;   // hole left by the device decode
+    if (slot == ~0ull) { atomicAdd(a.counters + 0, 1ull); continue; }   // hole left by the device decode
       if (slot >= a.n_slots) { atomicAdd(a.counters + 4, 1ull); continue; }
     Scratch* s = a.scr + slot;
     uint32_t fl, mode[W], val[W];

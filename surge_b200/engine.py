@@ -221,6 +221,14 @@ class ReplayEngine:
                                    C.byref(outlen), C.byref(exists)))
         return bytes(buf.raw[:outlen.value]) if exists.value else None
 
+    def index_of(self, key: str) -> Optional[int]:
+        """Dense aggregate index `get(key)` reads, or None for an unknown id."""
+        kb = key.encode("utf-8")
+        kbuf = C.create_string_buffer(kb, len(kb)) if kb else None
+        agg = C.c_uint64()
+        self._ck(self._lib.sgr_key_index(self._h, C.cast(kbuf, C.c_void_p) if kbuf else None, len(kb), C.byref(agg)))
+        return None if agg.value == (1 << 64) - 1 else int(agg.value)
+
     def get_index(self, agg: int) -> Tuple[Optional[bytes], int, int]:
         """(program bytes or None, flags, err_idx) of one dense aggregate index."""
         buf = C.create_string_buffer(N.MAX_STATE_BYTES)

@@ -115,6 +115,7 @@ ABI = [
     ("sgr_get", C.c_int32, [_P, _P, C.c_uint32, _P, C.c_uint32, C.POINTER(C.c_uint32), C.POINTER(C.c_int32)]),
     ("sgr_get_index", C.c_int32, [_P, C.c_uint64, _P, C.c_uint32, C.POINTER(C.c_uint32), C.POINTER(C.c_int32),
                                   C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
+    ("sgr_key_index", C.c_int32, [_P, _P, C.c_uint32, C.POINTER(C.c_uint64)]),
     ("sgr_export_states", C.c_int32, [_P, _P, C.c_uint64, _P, _P, _P]),
     ("sgr_states_device", C.c_int32, [_P, C.POINTER(_P), C.POINTER(C.c_uint64), C.POINTER(C.c_uint32)]),
     ("sgr_events_device", C.c_int32, [_P, C.POINTER(_P), C.POINTER(C.c_uint64), C.POINTER(_P)]),
